@@ -306,6 +306,27 @@ def test_bench_roofline_block_is_serialisable(path, tile, trtri):
     assert bench.roofline_block(args, path, timers, None, 35.5, flops, timers["var"], 24.0, n, variant=tile)["frac"] is None
 
 
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: the caller's arrays of the last step as float64 .npy files, every test point while they
+    fit the size limit, beyond it the same seeded sample in every run."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    if root not in sys.path:
+        sys.path.insert(0, root)
+    import bench
+    m = 1000
+    mean, var = np.linspace(-2.0, 3.0, m), np.linspace(0.0, 1.0, m)
+    bench.dump_outputs(str(tmp_path / "out"), mean, var, -1.5, 0, m, 0, 1)
+    for name, want in (("mean", mean), ("var", var), ("logp", [-1.5])):
+        got = np.load(tmp_path / "out" / (name + ".npy"))
+        assert got.dtype == np.float64
+        np.testing.assert_array_equal(got, want)
+    big = bench.DUMP_LIMIT // 8
+    idx = bench.dump_index(big)
+    assert 0.99 * bench.DUMP_LIMIT < 16 * len(idx) < bench.DUMP_LIMIT - 1024
+    assert np.all(np.diff(idx) > 0) and idx[-1] < big
+    np.testing.assert_array_equal(idx, bench.dump_index(big))
+
+
 def _load_protocol_sim(mutate=None):
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     src = open(os.path.join(root, "tools", "oz_protocol_sim.py")).read()
