@@ -51,6 +51,29 @@ GPR <- R6::R6Class("GPR",
       Ks <- covariance_matrix(private$.X, X_star, private$.k)
       v <- .Call(C_gprc_gpr_get, private$.ptr, 2L) %*% Ks            # L^-1 K_star
       list(t(Ks) %*% self$alpha, covariance_matrix(X_star, X_star, private$.k) - t(v) %*% v)
+    },
+    # append training points in place: afterwards the model is GPR$new(cbind(X, X_new), c(y, y_new), noise, k) with
+    # this model's noise and kernel.  Built-in kernels extend the Cholesky factor on the device; a matrix that is not
+    # positive definite with this noise, or a closure kernel, takes the constructor's path (noise-bump loop included).
+    add_points = function(X_new, y_new) {
+      stopifnot(is.numeric(X_new), length(X_new) %% nrow(private$.X) == 0)
+      if (is.null(dim(X_new))) dim(X_new) <- c(nrow(private$.X), length(X_new) / nrow(private$.X))
+      if (nrow(X_new) != nrow(private$.X)) stop("non-conformable arrays")
+      stopifnot(is.numeric(y_new), is.vector(y_new), length(y_new) == ncol(X_new))
+      if (ncol(X_new) == 0) return(invisible(self))
+      storage.mode(X_new) <- "double"
+      X <- cbind(private$.X, X_new); y <- c(private$.y, y_new)
+      if (!is.null(.gprc_spec(private$.k))) {
+        res <- .Call(C_gprc_gpr_append, private$.ptr, X_new, as.double(y_new))   # list(logp, info)
+        if (res[[2]] == 0 && is.finite(res[[1]])) {
+          private$.X <- X; private$.y <- y; private$.logp <- matrix(res[[1]], 1, 1)
+          return(invisible(self))
+        }
+      }
+      fresh <- GPR$new(X, y, private$.noise, private$.k)$.__enclos_env__$private
+      private$.X <- fresh$.X; private$.y <- fresh$.y; private$.ptr <- fresh$.ptr
+      private$.noise <- fresh$.noise; private$.logp <- fresh$.logp
+      invisible(self)
     }
   ),
   active = list(

@@ -77,6 +77,7 @@ SIGNATURES = {
                                    c_long_p]),
     "gprc_gpr_fit_precomputed": (C.c_int, [_P, c_double_p, C.c_long, c_double_p, C.c_double, C.POINTER(_P),
                                            c_double_p, c_long_p]),
+    "gprc_gpr_append": (C.c_int, [_P, c_double_p, C.c_long, c_double_p, c_double_p, c_long_p]),
     "gprc_gpr_predict": (C.c_int, [_P, c_double_p, C.c_long, c_double_p, c_double_p]),
     "gprc_gpr_predict_dev": (C.c_int, [_P, _P, C.c_long, _P, _P]),
     "gprc_gpr_predict_precomputed": (C.c_int, [_P, c_double_p, c_double_p, C.c_long, c_double_p, c_double_p]),

@@ -1287,6 +1287,179 @@ extern "C" int gprc_gpr_fit_precomputed(gprc_ctx* c, const double* K, long n, co
   return gpr_fit_common(c, nullptr, nullptr, false, 0, n, y, false, K, noise, out, logp, info, nullptr);
 }
 
+// Append k training points in place.  The leading n0 x n0 block of the factor (n0 = 128 floor(n / 128)) stays valid;
+// rows n0 .. n + k - 1 -- the old partial block row plus the new points, k' <= k + 127 of them -- are recomputed, so that
+// every step works on 128-aligned blocks:
+//   build  L[n0:, :n0] = K(X_new', X[:, :n0]),  L[n0:, n0:] = K(X_new', X_new') + noise I   (X_new' = points n0 ..)
+//   solve  L[n0:, :n0] <- L[n0:, :n0] L11^-T      trsm_flow_kernel
+//   Schur  L[n0:, n0:] -= L[n0:, :n0] L[n0:, :n0]^T  SyrkPolicy on the lower tiles
+//   factor L[n0:, n0:] in place                  potrf_blocked (inverted diagonal blocks and diag come with it)
+// then alpha and logp over the whole new factor as in gpr_finish_fit.  Costs n0^3 / 3 flops less than a refit.
+// When n + k outgrows the padding, every buffer is reallocated at round_up(n + k, 128) and L[:n0, :n0] is copied over
+// (the old buffers are released only once the new factor is complete).  Otherwise the rows that are overwritten -- the old
+// block row n0 / 128, its inverted diagonal block and diagonal entries -- are saved first: on info > 0 they are put back,
+// so a failed append leaves the model exactly as it was.  Derived state (W = L^-1, the INT8 digit planes, the predict
+// workspace) is dropped on success and rebuilt by the next predict that needs it.
+extern "C" int gprc_gpr_append(gprc_gpr* g, const double* Xnew, long k, const double* ynew, double* logp, long* info) {
+  GPRC_ARG(g && Xnew && ynew && logp && info && k > 0);
+  GPRC_ARG(!g->precomputed);  // closure kernels: the host refits with K built from the closure
+  gprc_ctx* c = g->ctx;
+  DeviceGuard guard(c);
+  *info = 0;
+  FactorState& F = g->F;
+  const int d = g->d;
+  const long n = F.n, n1 = n + k, n0 = n / NB * NB;
+  const bool grow = round_up(n1, NB) > F.n_pad;
+  const long ld = grow ? round_up(n1, NB) : F.n_pad;  // leading dimension = padded order, as everywhere
+  const long rows = ld - n0;                          // rows recomputed, padding included
+  double *X = nullptr, *L = F.L, *dinv = F.dinv, *diag = F.diag, *y = g->y, *alpha = g->alpha;
+  double *save = nullptr, *work = nullptr, *tmp = nullptr;
+  int* sched = nullptr;
+  bool restore = false;
+  int rc = 0;
+  do {
+    if ((rc = dmalloc(&X, (size_t)d * n1))) break;
+    cudaMemcpyAsync(X, g->X, sizeof(double) * d * n, cudaMemcpyDeviceToDevice, c->stream);
+    cudaMemcpyAsync(X + d * n, Xnew, sizeof(double) * d * k, cudaMemcpyHostToDevice, c->stream);
+    if (grow) {
+      L = dinv = diag = y = alpha = nullptr;
+      if ((rc = dmalloc(&L, (size_t)ld * ld))) break;
+      if ((rc = dmalloc(&dinv, (size_t)ld * NB))) break;
+      if ((rc = dmalloc(&diag, (size_t)ld))) break;
+      if ((rc = dmalloc(&y, (size_t)ld))) break;
+      if ((rc = dmalloc(&alpha, (size_t)ld))) break;
+      if (n0 > 0) {
+        cudaMemcpy2DAsync(L, ld * sizeof(double), F.L, F.n_pad * sizeof(double), n0 * sizeof(double), n0,
+                          cudaMemcpyDeviceToDevice, c->stream);
+        cudaMemcpyAsync(dinv, F.dinv, sizeof(double) * n0 * NB, cudaMemcpyDeviceToDevice, c->stream);
+        cudaMemcpyAsync(diag, F.diag, sizeof(double) * n0, cudaMemcpyDeviceToDevice, c->stream);
+      }
+      cudaMemsetAsync(y, 0, sizeof(double) * ld, c->stream);
+      cudaMemcpyAsync(y, g->y, sizeof(double) * n, cudaMemcpyDeviceToDevice, c->stream);
+    } else {
+      // block row n0 / 128 (all ld columns), then its inverted diagonal block and its diagonal entries
+      if ((rc = dmalloc(&save, (size_t)NB * ld + NB * NB + NB))) break;
+      cudaMemcpy2DAsync(save, NB * sizeof(double), L + n0, ld * sizeof(double), NB * sizeof(double), ld,
+                        cudaMemcpyDeviceToDevice, c->stream);
+      cudaMemcpyAsync(save + NB * ld, dinv + n0 * NB, sizeof(double) * NB * NB, cudaMemcpyDeviceToDevice, c->stream);
+      cudaMemcpyAsync(save + NB * ld + NB * NB, diag + n0, sizeof(double) * NB, cudaMemcpyDeviceToDevice, c->stream);
+      restore = true;
+    }
+    cudaMemcpyAsync(y + n, ynew, sizeof(double) * k, cudaMemcpyHostToDevice, c->stream);
+    {
+      PhaseTimer t(c, GPRC_T_BUILD_K);
+      if (n0 > 0 && (rc = cov_build_dev(c, g->spec.dev, X + d * n0, d, n1 - n0, X, n0, L + n0, ld, rows, n0, false, false,
+                                        0.0, false, nullptr, nullptr, nullptr, 0)))
+        break;
+      if ((rc = cov_build_dev(c, g->spec.dev, X + d * n0, d, n1 - n0, X + d * n0, n1 - n0, L + n0 + n0 * ld, ld, rows,
+                              rows, true, true, g->noise, true, nullptr, nullptr, nullptr, 0)))
+        break;
+    }
+    *c->h_info = LONG_MAX;
+    cudaMemcpyAsync(c->d_info, c->h_info, sizeof(long), cudaMemcpyHostToDevice, c->stream);
+    {
+      PhaseTimer t(c, GPRC_T_CHOL);
+      if (n0 > 0) {
+        if ((rc = dmalloc(&sched, (size_t)(rows / NB + 4)))) break;
+        if ((rc = trsm_flow(c, L, ld, dinv, (int)(n0 / NB), L + n0, ld, rows, sched))) break;
+        const long t1 = rows / NB;
+        SyrkPolicy sp{L, ld, 1, (int)(n0 / NB), 0, (int)n0};
+        if ((rc = launch_gemm(c, sp, dim3((unsigned)(t1 * (t1 + 1) / 2))))) break;
+      }
+      if ((rc = potrf_blocked(c, L + n0 + n0 * ld, rows, ld, dinv + n0 * NB, c->d_info, diag + n0))) break;
+    }
+    int* h_error = reinterpret_cast<int*>(c->h_scalars + 8);  // pinned
+    *h_error = 0;
+    if (sched) cudaMemcpyAsync(h_error, sched + 2, sizeof(int), cudaMemcpyDeviceToHost, c->stream);
+    cudaMemcpyAsync(c->h_info, c->d_info, sizeof(long), cudaMemcpyDeviceToHost, c->stream);
+    cudaError_t e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess) {
+      rc = set_error(-2, __FILE__, __LINE__, cudaGetErrorString(e));
+      break;
+    }
+    if (*h_error) {
+      rc = set_error(-6, __FILE__, __LINE__, "triangular solve of the appended rows: a block dependency never arrived");
+      break;
+    }
+    if (*c->h_info != LONG_MAX) {
+      *info = n0 + *c->h_info;
+      break;
+    }
+    // alpha and logp over the whole new factor
+    if ((rc = dmalloc(&work, (size_t)ld))) break;
+    if ((rc = dmalloc(&tmp, (size_t)ld))) break;
+    {
+      PhaseTimer t(c, GPRC_T_SOLVE);
+      if ((rc = potrs_vec(c, L, ld, ld, dinv, y, work, tmp, alpha))) break;
+      gp_reduce_kernel<<<1, 1024, 0, c->stream>>>(y, alpha, diag, n1, c->d_scalars);
+      c->launches++;
+    }
+    cudaMemcpyAsync(c->h_scalars, c->d_scalars, 4 * sizeof(double), cudaMemcpyDeviceToHost, c->stream);
+    e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess) {
+      rc = set_error(-2, __FILE__, __LINE__, cudaGetErrorString(e));
+      break;
+    }
+    restore = false;
+  } while (0);
+  dfree(sched);
+  dfree(work);
+  dfree(tmp);
+  if (rc != 0 || *info != 0) {
+    if (restore) {  // the old block row, its inverted diagonal block and diagonal; y's padding back to zero
+      cudaMemcpy2DAsync(L + n0, ld * sizeof(double), save, NB * sizeof(double), NB * sizeof(double), ld,
+                        cudaMemcpyDeviceToDevice, c->stream);
+      cudaMemcpyAsync(dinv + n0 * NB, save + NB * ld, sizeof(double) * NB * NB, cudaMemcpyDeviceToDevice, c->stream);
+      cudaMemcpyAsync(diag + n0, save + NB * ld + NB * NB, sizeof(double) * NB, cudaMemcpyDeviceToDevice, c->stream);
+      cudaMemsetAsync(y + n, 0, sizeof(double) * (F.n_pad - n), c->stream);
+    }
+    if (grow) {
+      dfree(L);
+      dfree(dinv);
+      dfree(diag);
+      dfree(y);
+      dfree(alpha);
+    }
+    dfree(X);
+    dfree(save);
+    cudaError_t e = cudaStreamSynchronize(c->stream);
+    if (rc == 0 && e != cudaSuccess) rc = set_error(-2, __FILE__, __LINE__, cudaGetErrorString(e));
+    return rc;
+  }
+  dfree(save);
+  if (grow) {
+    dfree(F.L);
+    dfree(F.dinv);
+    dfree(F.diag);
+    dfree(g->y);
+    dfree(g->alpha);
+    F.L = L;
+    F.dinv = dinv;
+    F.diag = diag;
+    F.n_pad = ld;
+    g->y = y;
+    g->alpha = alpha;
+  }
+  dfree(g->X);
+  g->X = X;
+  F.n = n1;
+  // derived from the old factor: rebuilt on demand by the next predict
+  dfree(F.W);
+  dfree(F.ozLs);
+  dfree(F.oz_erow);
+  dfree(F.oz_srow);
+  F.W = nullptr;
+  F.ozLs = nullptr;
+  F.oz_erow = nullptr;
+  F.oz_srow = nullptr;
+  F.oz_digits = 0;
+  g->ws.release();
+  // -0.5 * y %*% alpha - sum(log(diag(L))) - n / 2 * log(2 * pi)        R/GPRclass.R:153
+  g->logp = -0.5 * c->h_scalars[0] - c->h_scalars[1] - (double)n1 / 2.0 * log(2.0 * M_PI);
+  *logp = g->logp;
+  return 0;
+}
+
 extern "C" int gprc_gpr_predict_dev(gprc_gpr* g, const double* dXs, long m, double* dmean, double* dvar) {
   GPRC_ARG(g && dXs && dmean && dvar && m >= 0);
   GPRC_ARG(!g->precomputed);

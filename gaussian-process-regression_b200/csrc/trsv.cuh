@@ -9,6 +9,7 @@
 #include <cstring>
 
 #include "gemm.cuh"
+#include "potrf.cuh"  // chol_wait_progress: the watchdog of the persistent kernels
 
 namespace gprc {
 
@@ -422,6 +423,206 @@ inline int potrs_vec(gprc_ctx* ctx, const double* L, long n, long ld, const doub
   }
   return 0;
 }
+
+// ---------------------------------------------------------------------------------------------------------------
+// Triangular solve with a few hundred right-hand sides, as ONE dataflow kernel (the append of training points,
+// gprc_gpr_append):  T <- T L^-T  for a panel T of `rows` right-hand sides over the leading 128 nt columns of a factor L.
+// T is stored like K_star^T (right-hand side r, column c at T[r + c ldt]); in the append it is the new block row of L
+// itself.  Work unit (i, g) = block row i of L, group g of 128 right-hand sides:
+//     C = T_i[g] - sum_{j<i} L[i, j] V_j[g]      (DMMA GEMM, K = 128 i; TrsmLeftUpdatePolicy's epilogue)
+//     V_i[g] = Linv_i C                          (DMMA GEMM, K = 128, in place)
+// The substitution kernels of the predictive variance (TrsmLeft*Policy, trsm_persistent_kernel) run unit (i, g) only once
+// unit (i - 1, g) is complete, so one group of right-hand sides keeps ONE SM busy for all nt (nt + 1) / 2 tile products.
+// Here the units are handed out i-major by an atomic counter and every unit streams in block j of its GEMM as soon as
+// group g's block row j is published (progress[g] >= j + 1, release / acquire, checked by the producer lane per 128-wide
+// k-block): the units of one group run on different SMs and overlap, and the critical path per block row is the product
+// with the tile next to the diagonal (prefetched into L2 when the unit starts) plus the product with Linv_i.  All groups
+// run in the same launch.  Every prerequisite of a unit has a smaller index and units only go to running CTAs, so no
+// co-residency is needed; a dependency that never arrives sets `error` (chol_wait_progress) and the host reports it.
+// Summation orders are fixed: bitwise reproducible.
+// ---------------------------------------------------------------------------------------------------------------
+struct TrsmFlowParams {
+  const double* L;
+  long ldl;
+  const double* dinv;
+  double* T;
+  long ldt;
+  int nt, ngroups;
+  unsigned long long* next;  // unit counter (zeroed by the host)
+  int* error;                // watchdog (zeroed by the host)
+  int* progress;             // [ngroups] block rows published per group (zeroed by the host)
+};
+
+__global__ void __launch_bounds__(GEMM_THREADS, 1) trsm_flow_kernel(const TrsmFlowParams p) {
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  double* smem = reinterpret_cast<double*>(smem_raw);
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + STAGES * STAGE_DOUBLES * 8);
+  uint64_t* empty = full + STAGES;
+  __shared__ long long s_item;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x == 0) {
+#pragma unroll
+    for (int s = 0; s < STAGES; ++s) {
+      mbar_init(smem_u32(full + s), 1);
+      mbar_init(smem_u32(empty + s), GEMM_CONSUMERS / 32);
+    }
+    mbar_fence_init();
+  }
+  __syncthreads();
+  const long long total = (long long)p.nt * p.ngroups;
+  long long base = 0;  // k-slices pushed through the ring so far (identical for producer and consumers)
+  const WarpCoord wc;
+  for (;;) {
+    if (threadIdx.x == 0) {
+      long long item = (long long)atomicAdd(p.next, 1ULL);
+      if (*reinterpret_cast<volatile int*>(p.error)) item = total;
+      s_item = item;
+    }
+    __syncthreads();
+    const long long item = s_item;
+    if (item >= total) break;
+    const int g = (int)(item % p.ngroups), i = (int)(item / p.ngroups);
+    double* Ctile = p.T + (long)g * NB + (long)i * NB * p.ldt;  // element (m, n) of the tile at C[n + m * ldt]
+    // ---- phase 0: C -= sum_{j<i} L[i, j] V_j, block j as soon as it is published ----
+    {
+      TileWork w;
+      w.A = p.L + (long)i * NB;
+      w.lda = p.ldl;
+      w.B = p.T + (long)g * NB;  // element (k, n) = V[k, n] = T[n + k * ldt]
+      w.ldb = p.ldt;
+      w.k_begin = 0;
+      w.k_end = i * NB;
+      const int KT = i * (NB / BK);
+      if (warp == GEMM_CONSUMERS / 32) {
+        if (lane == 0) {
+          bool ok = true;
+          for (int kt = 0; kt < KT; ++kt) {
+            if (kt % (NB / BK) == 0) {
+              ok = ok && chol_wait_progress(p.progress + g, kt / (NB / BK) + 1, p.error);
+              fence_proxy_async();  // V_j was written with ordinary stores and is read by the TMA engine
+            }
+            const long long gk = base + kt;
+            const int s = (int)(gk % STAGES);
+            if (gk >= STAGES) mbar_wait(smem_u32(empty + s), (uint32_t)(((gk / STAGES) - 1) & 1));
+            if (ok) produce_stage<false>(w, kt * BK, smem + s * STAGE_DOUBLES, smem_u32(full + s));
+            else mbar_arrive(smem_u32(full + s));  // watchdog fired: release the consumers (results are garbage, error set)
+          }
+        }
+      } else if (KT > 0) {
+        Acc acc;
+#pragma unroll
+        for (int mb = 0; mb < 8; ++mb)
+#pragma unroll
+          for (int nb = 0; nb < 4; ++nb) acc[mb][nb][0] = acc[mb][nb][1] = 0.0;
+        // the C tile, the tile next to the diagonal and Linv_i: everything the critical path reads after the last poll
+        const double* Lnext = p.L + (long)i * NB + (long)(i - 1) * NB * p.ldl;
+        const double* Li = p.dinv + (long)i * NB * NB;
+#pragma unroll
+        for (int qq = 0; qq < 4; ++qq) {
+          const int line = threadIdx.x + qq * GEMM_CONSUMERS;
+          prefetch_l2(Ctile + (long)(line >> 3) * p.ldt + (line & 7) * 16);
+          prefetch_l2(Lnext + (long)(line >> 3) * p.ldl + (line & 7) * 16);
+          prefetch_l2(Li + (long)line * 16);
+        }
+        for (int kt = 0; kt < KT; ++kt) {
+          const long long gk = base + kt;
+          const int s = (int)(gk % STAGES);
+          mbar_wait(smem_u32(full + s), (uint32_t)((gk / STAGES) & 1));
+          compute_stage<false>(smem + s * STAGE_DOUBLES, wc, acc);
+          __syncwarp();
+          if (lane == 0) mbar_arrive(smem_u32(empty + s));
+        }
+        TrsmLeftUpdatePolicy pol{p.L, p.ldl, p.T, p.ldt, i};
+        TrsmLeftUpdatePolicy::Tile tile{Ctile};
+        pol.epilogue(tile, acc, smem);
+        __threadfence();
+        fence_proxy_async();  // phase 1 reads C through the TMA engine
+      }
+      __syncthreads();
+      base += KT;
+    }
+    // ---- phase 1: V_i = Linv_i C, in place ----
+    {
+      TileWork w;
+      w.A = p.dinv + (long)i * NB * NB;
+      w.lda = NB;
+      w.B = Ctile;  // element (k, n) = C[k, n]
+      w.ldb = p.ldt;
+      w.k_begin = 0;
+      w.k_end = NB;
+      constexpr int KT = NB / BK;
+      if (warp == GEMM_CONSUMERS / 32) {
+        if (lane == 0) {
+          fence_proxy_async();
+          for (int kt = 0; kt < KT; ++kt) {
+            const long long gk = base + kt;
+            const int s = (int)(gk % STAGES);
+            if (gk >= STAGES) mbar_wait(smem_u32(empty + s), (uint32_t)(((gk / STAGES) - 1) & 1));
+            produce_stage<false>(w, kt * BK, smem + s * STAGE_DOUBLES, smem_u32(full + s));
+          }
+        }
+      } else {
+        Acc acc;
+#pragma unroll
+        for (int mb = 0; mb < 8; ++mb)
+#pragma unroll
+          for (int nb = 0; nb < 4; ++nb) acc[mb][nb][0] = acc[mb][nb][1] = 0.0;
+        for (int kt = 0; kt < KT; ++kt) {
+          const long long gk = base + kt;
+          const int s = (int)(gk % STAGES);
+          mbar_wait(smem_u32(full + s), (uint32_t)((gk / STAGES) & 1));
+          compute_stage<false>(smem + s * STAGE_DOUBLES, wc, acc);
+          __syncwarp();
+          if (lane == 0) mbar_arrive(smem_u32(empty + s));
+        }
+        // every k-slice of C has landed in shared memory (this warp passed the last full barrier): overwrite C by V_i
+#pragma unroll
+        for (int mb = 0; mb < 8; ++mb) {
+          double* cp = Ctile + (long)wc.row(mb) * p.ldt;
+#pragma unroll
+          for (int nb = 0; nb < 4; ++nb)
+            *reinterpret_cast<double2*>(cp + wc.col(nb, 0)) = make_double2(acc[mb][nb][0], acc[mb][nb][1]);
+        }
+        __threadfence();
+        fence_proxy_async();  // the next units read V_i through the TMA engine
+      }
+      __syncthreads();
+      base += KT;
+    }
+    if (threadIdx.x == 0) st_release_gpu(p.progress + g, i + 1);
+  }
+}
+
+// T <- T L^-T for `rows` right-hand sides (T: round_up(rows, 128) x 128 nt, leading dimension ldt; the padding rows are
+// solved too and must hold finite values).  sched: ngroups + 4 ints of device scratch.
+inline int trsm_flow(gprc_ctx* ctx, const double* L, long ldl, const double* dinv, int nt, double* T, long ldt, long rows,
+                     int* sched) {
+  static bool configured[64] = {false};
+  if (!configured[ctx->device & 63]) {
+    GPRC_CUDA(cudaFuncSetAttribute(trsm_flow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+    configured[ctx->device & 63] = true;
+  }
+  const int ngroups = (int)((rows + NB - 1) / NB);
+  if (nt <= 0 || ngroups <= 0) return 0;
+  GPRC_CUDA(cudaMemsetAsync(sched, 0, sizeof(int) * (ngroups + 4), ctx->stream));
+  TrsmFlowParams p;
+  p.L = L;
+  p.ldl = ldl;
+  p.dinv = dinv;
+  p.T = T;
+  p.ldt = ldt;
+  p.nt = nt;
+  p.ngroups = ngroups;
+  p.next = reinterpret_cast<unsigned long long*>(sched);
+  p.error = sched + 2;
+  p.progress = sched + 4;
+  const int grid = (int)std::min<long>((long)nt * ngroups, ctx->sm_count);
+  trsm_flow_kernel<<<grid, GEMM_THREADS, GEMM_SMEM_BYTES, ctx->stream>>>(p);
+  ctx->launches++;
+  GPRC_CUDA(cudaGetLastError());
+  return 0;
+}
+
 // y = K^T v for a column-major n x n matrix (K symmetric in the callers): warp per column, coalesced.
 __global__ void __launch_bounds__(256) gemv_t_kernel(const double* __restrict__ K, long ld, long n,
                                                      const double* __restrict__ v, double* __restrict__ y) {

@@ -191,6 +191,51 @@ class GPR:
             cov = host_covariance_matrix(X_star, X_star, self._k) - v.T @ v
         return [mean.reshape(-1, 1), cov]
 
+    def add_points(self, X_new, y_new):
+        """Append training points in place and return the model: afterwards it is GPR(cbind(X, X_new), c(y, y_new),
+        noise = self.noise, k = self.k) (the kernel is kept, never re-fitted).  X_new follows predict's reshape rule.
+        Built-in kernels extend the existing Cholesky factor on the device (gprc_gpr_append); if the enlarged matrix is
+        not positive definite with this noise, or the kernel is a closure, the constructor's path runs on the
+        concatenated data (noise-bump loop from self.noise, same warning and error)."""
+        X_new = np.asarray(X_new)
+        y_new = np.asarray(y_new)
+        D = self._X.shape[0]
+        if not np.issubdtype(X_new.dtype, np.number) or X_new.size % D != 0:
+            raise ValueError("is.numeric(X_new), length(X_new) %% nrow(self$X) == 0 are not all TRUE")
+        X_new = X_new.astype(np.float64)
+        if X_new.ndim < 2:
+            X_new = X_new.reshape(-1, D).T  # dim(X_new) <- c(D, length / D)  (column-major fill)
+        elif X_new.ndim != 2 or X_new.shape[0] != D:
+            raise ValueError("non-conformable arrays: nrow(X_new) = %d, nrow(self$X) = %d" % (X_new.shape[0], D))
+        m = X_new.shape[1]
+        if not (np.issubdtype(y_new.dtype, np.number) and y_new.ndim == 1 and len(y_new) == m):
+            raise ValueError("is.numeric(y_new), is.vector(y_new), length(y_new) == ncol(X_new) are not all TRUE")
+        if m == 0:
+            return self
+        X_all = np.concatenate([self._X, X_new], axis=1)
+        y_all = np.concatenate([self._y, y_new.astype(np.float64)])
+        if kernel_spec_of(self._k) is not None:
+            lib = self._ctx.lib
+            xp = _lib.points(X_new)
+            yp = np.ascontiguousarray(y_new, dtype=np.float64)
+            logp = C.c_double(0.0)
+            info = C.c_long(0)
+            _lib.check(lib.gprc_gpr_append(self._handle, _lib.dptr(xp), m, _lib.dptr(yp), C.byref(logp),
+                                           C.byref(info)))
+            if info.value == 0 and np.isfinite(logp.value):
+                self._X, self._y = X_all, y_all
+                self._logp = np.array([[logp.value]])
+                self._alpha = None
+                self._L = None
+                return self
+        fresh = GPR(X_all, y_all, noise=self._noise, k=self._k, ctx=self._ctx)
+        self._ctx.lib.gprc_gpr_free(self._handle)
+        self._handle, fresh._handle = fresh._handle, None
+        self._X, self._y, self._noise, self._logp = fresh._X, fresh._y, fresh._noise, fresh._logp
+        self._alpha = None
+        self._L = None
+        return self
+
 
 def _fmt(x):
     return ("%.15g" % x)

@@ -128,6 +128,23 @@ SEXP C_gprc_gpr_predict_cov(SEXP ptr, SEXP Xs) {
   return out;
 }
 
+/* $add_points(X_new, y_new) of built-in kernels: list(logp, info); info > 0 leaves the model as it was */
+SEXP C_gprc_gpr_append(SEXP ptr, SEXP Xnew, SEXP ynew) {
+  gprc_gpr* g = (gprc_gpr*)R_ExternalPtrAddr(ptr);
+  if (!g) Rf_error("gprc: model handle is NULL");
+  const long k = Rf_ncols(Xnew);
+  /* the library reads d x k and k doubles */
+  if (Rf_nrows(Xnew) != gprc_gpr_dim(g) || XLENGTH(ynew) != k) Rf_error("non-conformable arrays");
+  double logp = NA_REAL; long info = 0;
+  int rc = gprc_gpr_append(g, REAL(Xnew), k, REAL(ynew), &logp, &info);
+  if (rc) Rf_error("gprc: %s", gprc_last_error());
+  SEXP out = PROTECT(Rf_allocVector(VECSXP, 2));
+  SET_VECTOR_ELT(out, 0, Rf_ScalarReal(logp));
+  SET_VECTOR_ELT(out, 1, Rf_ScalarReal((double)info));
+  UNPROTECT(1);
+  return out;
+}
+
 /* active bindings $L / $alpha (lazy download), R/GPRclass.R:258-273 */
 SEXP C_gprc_gpr_get(SEXP ptr, SEXP what) {
   gprc_gpr* g = (gprc_gpr*)R_ExternalPtrAddr(ptr);
@@ -265,6 +282,7 @@ static const R_CallMethodDef call_methods[] = {
     {"C_gprc_gpr_fit", (DL_FUNC)&C_gprc_gpr_fit, 5},
     {"C_gprc_gpr_predict", (DL_FUNC)&C_gprc_gpr_predict, 4},
     {"C_gprc_gpr_predict_cov", (DL_FUNC)&C_gprc_gpr_predict_cov, 2},
+    {"C_gprc_gpr_append", (DL_FUNC)&C_gprc_gpr_append, 3},
     {"C_gprc_gpr_get", (DL_FUNC)&C_gprc_gpr_get, 2},
     {"C_gprc_logml", (DL_FUNC)&C_gprc_logml, 4},
     {"C_gprc_logml_grad", (DL_FUNC)&C_gprc_logml_grad, 6},

@@ -161,6 +161,12 @@ int gprc_gpr_fit_dev(gprc_ctx* ctx, const gprc_kernel* k, const double* dX, int 
 /* k is an arbitrary closure evaluated by the host: K (n x n, no noise added yet) comes in precomputed. */
 int gprc_gpr_fit_precomputed(gprc_ctx* ctx, const double* K, long n, const double* y, double noise, gprc_gpr** out,
                              double* logp, long* info);
+/* Append k training points (Xnew: d x k, points contiguous; ynew: k) to a fitted model, in place.  Afterwards the
+ * model is what gprc_gpr_fit gives for cbind(X, Xnew), c(y, ynew) with the model's noise (the possibly bumped one),
+ * up to rounding.  *logp receives the new log marginal likelihood.  info > 0: the enlarged K + noise I is not positive
+ * definite (1-based row); the model is left exactly as it was.  Built-in kernels only: a closure-kernel
+ * (precomputed) model returns an argument error. */
+int gprc_gpr_append(gprc_gpr* g, const double* Xnew, long k, const double* ynew, double* logp, long* info);
 /* GPR$predict(X_star, pointwise_var = TRUE), R/GPRclass.R:155-165: mean (m), var (m). */
 int gprc_gpr_predict(gprc_gpr* g, const double* Xs, long m, double* mean, double* var);
 int gprc_gpr_predict_dev(gprc_gpr* g, const double* dXs, long m, double* dmean, double* dvar);
