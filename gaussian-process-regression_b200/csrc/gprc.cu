@@ -2487,16 +2487,21 @@ extern "C" int gprc_dev_trtri(gprc_ctx* c, const double* dL, long n, long ld, co
 // posterior sampling helper: multivariate_normal(), R/GPRclass.R:360-370
 // =================================================================================================================
 namespace gprc {
+// Both kernels stride over the columns by gridDim.y: launched on grid_cols() they take any number of columns, where one
+// column per grid row would stop at the 65 535 limit of gridDim.y (more draws than that, or a wider covariance).
+constexpr long MAX_GRID_Y = 65535;
+static inline dim3 grid_cols(long rows, long cols) { return grid2(rows, std::min(cols, MAX_GRID_Y)); }
 // zero everything strictly above the diagonal (the uploaded covariance had both triangles)
 __global__ void tril_inplace_kernel(double* __restrict__ M, long ld, long n) {
   const long i = blockIdx.x * (long)blockDim.x + threadIdx.x;
-  const long j = blockIdx.y;
-  if (i < n && j < n && i < j) M[i + j * ld] = 0.0;
+  if (i >= n) return;
+  for (long j = i + 1 + blockIdx.y; j < n; j += gridDim.y) M[i + j * ld] = 0.0;
 }
 __global__ void add_mean_kernel(double* __restrict__ out, long ld, long m, long ns, const double* __restrict__ mean) {
   const long i = blockIdx.x * (long)blockDim.x + threadIdx.x;
-  const long j = blockIdx.y;
-  if (i < m && j < ns) out[i + j * ld] += mean[i];
+  if (i >= m) return;
+  const double mu = mean[i];
+  for (long j = blockIdx.y; j < ns; j += gridDim.y) out[i + j * ld] += mu;
 }
 }  // namespace gprc
 
@@ -2507,6 +2512,11 @@ extern "C" int gprc_mvn_sample(gprc_ctx* c, const double* mean, const double* co
   FactorState F;
   double *dZ = nullptr, *dout = nullptr, *dmean = nullptr;
   const long sp = round_up(ns, NB);
+  // a failed launch is reported here and the buffers below are still released
+  auto launched = []() -> int {
+    GPRC_CUDA(cudaGetLastError());
+    return 0;
+  };
   int rc = 0;
   *info = 0;
   do {
@@ -2521,12 +2531,14 @@ extern "C" int gprc_mvn_sample(gprc_ctx* c, const double* mean, const double* co
     cudaMemcpy2DAsync(dZ, mp * sizeof(double), Z, m * sizeof(double), m * sizeof(double), ns, cudaMemcpyHostToDevice,
                       c->stream);
     cudaMemcpyAsync(dmean, mean, sizeof(double) * m, cudaMemcpyHostToDevice, c->stream);
-    tril_inplace_kernel<<<grid2(mp, mp), 256, 0, c->stream>>>(F.L, mp, mp);
+    tril_inplace_kernel<<<grid_cols(mp, mp), 256, 0, c->stream>>>(F.L, mp, mp);
     c->launches++;
+    if ((rc = launched())) break;
     DgemmPolicy<true> pol{F.L, mp, dZ, mp, dout, mp, 1.0, 0.0, (int)mp, (int)(mp / NB)};  // L %*% Z
     if ((rc = launch_gemm(c, pol, dim3((unsigned)((mp / NB) * (sp / NB)))))) break;
-    add_mean_kernel<<<grid2(m, ns), 256, 0, c->stream>>>(dout, mp, m, ns, dmean);
+    add_mean_kernel<<<grid_cols(m, ns), 256, 0, c->stream>>>(dout, mp, m, ns, dmean);
     c->launches++;
+    if ((rc = launched())) break;
     cudaMemcpy2DAsync(out, m * sizeof(double), dout, mp * sizeof(double), m * sizeof(double), ns, cudaMemcpyDeviceToHost,
                       c->stream);
     cudaError_t e = cudaStreamSynchronize(c->stream);
