@@ -6,8 +6,8 @@
   function(v) {
     spec <- c(list(id = .gprc_ids[[name]]), setNames(as.list(as.double(v)), .gprc_formals(name)))
     r <- .Call(C_gprc_logml, spec, X, as.double(y), as.double(noise))   # c(logp, min leading-minor log det, info)
-    # stopifnot(min(sapply(1:n, function(i) det(...[1:i, 1:i]))) > 0): det() = exp(log-modulus) is 0 below exp(-745)
-    if (r[3] != 0 || !is.finite(r[1]) || (strict && r[2] < log(.Machine$double.xmin * .Machine$double.eps)))
+    # stopifnot(min(sapply(1:n, function(i) det(...[1:i, 1:i]))) > 0): det() = exp(log-modulus), 0 below log(2^-1075)
+    if (r[3] != 0 || !is.finite(r[1]) || (strict && !(exp(r[2]) > 0)))
       stop("covariance matrix is not (numerically) positive definite")
     matrix(r[1], 1, 1)
   }

@@ -2020,7 +2020,6 @@ extern "C" int gprc_fit_family(gprc_ctx* c, int kernel_id, const double* X, int 
   cudaMemcpyAsync(dy, y, sizeof(double) * n, cudaMemcpyHostToDevice, c->stream);
   long n_fn = 0, n_gr = 0;
   int hard_error = 0;  // a CUDA / argument error inside an evaluation: abort the search and report it
-  const double log_denorm_min = std::log(std::numeric_limits<double>::denorm_min());
   // dens, R/fit.R:117-124
   auto dens = [&](const double* v) -> double {
     gprc_kernel k = family_spec(kernel_id, v);
@@ -2035,7 +2034,8 @@ extern "C" int gprc_fit_family(gprc_ctx* c, int kernel_id, const double* X, int 
       throw optim::ObjectiveError{};
     }
     if (inf != 0 || !std::isfinite(lp)) throw optim::ObjectiveError{};             // chol() failed
-    if (minors_rule == 0 && !(ml >= log_denorm_min)) throw optim::ObjectiveError{};  // fit.R:119 with det underflow (A.4)
+    // fit.R:119 with det() = exp(log-modulus), which underflows to 0 below log(2^-1075) (A.4)
+    if (minors_rule == 0 && !(std::exp(ml) > 0.0)) throw optim::ObjectiveError{};
     return lp;
   };
   const int nparam = (kernel_id == GPRC_GAMMAEXP || kernel_id == GPRC_RATQUAD || kernel_id == GPRC_POLYNOMIAL) ? 2 : 1;

@@ -25,7 +25,6 @@ cov_dict = {
     "rationalquadratic": dict(func=BUILTIN["rationalquadratic"], display="Rational Quadratic", start=[1.0, 1.0]),
 }
 HAS_DERIV = ("sqrexp", "gammaexp", "rationalquadratic", "polynomial")  # R/fit.R:125
-LOG_DBL_MIN_DENORM = math.log(5e-324)  # det() = exp(log-modulus) is 0 below this (SURVEY.md A.4)
 
 
 def _spec(name, v):
@@ -53,8 +52,9 @@ class Objective:
                                            C.byref(info)))
         if info.value != 0 or not math.isfinite(logp.value):
             raise OptimError("not positive definite (leading minor %d)" % info.value)
-        # R/fit.R:119: min over the leading minors of det(.) > 0; det underflows to 0 below exp(-745) (A.4)
-        if self.minors == "literal" and not (minlog.value >= LOG_DBL_MIN_DENORM):
+        # R/fit.R:119: min over the leading minors of det(.) > 0, with det() = exp(log-modulus), which rounds to 0 below
+        # log(2^-1075) = -745.13 (A.4): the same exp() decides here
+        if self.minors == "literal" and not (math.exp(minlog.value) > 0.0):
             raise OptimError("min(sapply(..., det)) > 0 is not TRUE")
         return logp.value
 
